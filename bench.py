@@ -2,7 +2,7 @@
 """Benchmark of the post-rollout NPG/TRPO/DAPG update path (BASELINE.json metric: train_step/s and FVP/s on a
 1e6-timestep batch).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg3] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg3] [--impl reference] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  A "step" = everything mjrl's train_step does after sampling
 (algos/batch_reinforce.py:94-112): returns -> baseline predict -> GAE -> whitening -> VPG -> 10-iteration CG
@@ -255,19 +255,25 @@ def run_reference(args, cfg, rank, world):
         full_s = time.time() - t0
         backtracks = r["backtracks"]
         del step_f
-    t0 = time.time()
-    k = max(1, args.steps - 1)
-    for _ in range(k):
-        step_s()
-    dt_s = (time.time() - t0) / k
+    k = args.steps - (full_s is not None)
+    dt_s = None
+    if k > 0:
+        t0 = time.time()
+        for _ in range(k):
+            step_s()
+        dt_s = (time.time() - t0) / k
     scale = (cfg["n_traj"] * cfg["horizon"]) / n
     sec_per_step = full_s if full_s is not None else dt_s * scale
     value = 1.0 / sec_per_step
     fvp_t = fvp_time() * scale
-    sample = ("1 timed step on the FULL batch (%d trajectories, %d timesteps, no extrapolation) = %.1f s; plus %d steps on "
-              "%d trajectories (%d timesteps) = %.2f s each, x%.0f = %.1f s extrapolated (cross-check only)"
-              % (n_full, n_full * cfg["horizon"], full_s, k, n_s, n, dt_s, scale, dt_s * scale)) if full_s is not None else \
-             ("%d of %d trajectories (%d timesteps) per step; extrapolated linearly x%.0f" % (n_s, cfg["n_traj"], n, scale))
+    if full_s is None:
+        sample = "%d of %d trajectories (%d timesteps) per step; extrapolated linearly x%.0f" % (n_s, cfg["n_traj"], n, scale)
+    else:
+        sample = "1 timed step on the FULL batch (%d trajectories, %d timesteps, no extrapolation) = %.1f s" % (
+            n_full, n_full * cfg["horizon"], full_s)
+        if dt_s is not None:
+            sample += ("; plus %d steps on %d trajectories (%d timesteps) = %.2f s each, x%.0f = %.1f s extrapolated "
+                       "(cross-check only)" % (k, n_s, n, dt_s, scale, dt_s * scale))
     line = {"impl": "reference", "metric": "train_step_per_sec", "value": value, "unit": "train_step/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": sec_per_step * 1e3, "higher_is_better": True,
             "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -275,7 +281,7 @@ def run_reference(args, cfg, rank, world):
             "trpo_backtracks_full_batch": backtracks,
             "cpu_baseline": {"value": value, "unit": "train_step/s", "cores": threads, "os_cpu_count": os.cpu_count(),
                              "kind": kind, "sample": sample, "thread_calibration_s_per_fvp": table,
-                             "extrapolated_from_sample_ms": dt_s * scale * 1e3},
+                             "extrapolated_from_sample_ms": None if dt_s is None else dt_s * scale * 1e3},
             "e2e": {"value": value, "unit": "train_step/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     print(json.dumps(line), flush=True)
 
@@ -347,6 +353,30 @@ def workload_config(cfg, args, world):
                            "gradient and the scalar statistics)" % world,
             "cache": "batch < L2 on purpose of the workload: obs stays L2-resident across the 10 CG FVPs of a step as in "
                      "production; every step also streams the 1e6-row fit gather + GAE arrays (> L2 in total)"}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, eng, st):
+    """Write what the timed path computed in its last step, as its caller receives it, to out_dir/<name>.npy: the
+    updated policy parameters, the step's vanilla and natural gradients and its statistics, the fitted baseline
+    weights, and the per-timestep returns, baseline predictions, GAE advantages and whitened advantages of the
+    resident batch (this rank's shard).  Every input is seeded, so two builds run with the same arguments can be
+    compared array by array."""
+    vpg, npg = eng.last_vectors()
+    out = {"policy_params": eng.get_params(), "vpg_grad": vpg, "npg_grad": npg, "baseline_weights": eng.vf_get_state()[0],
+           "returns": eng.returns(), "baseline": eng.baseline(), "advantages": eng.advantages(),
+           "adv_white": eng.adv_white(),
+           "step_stats": np.array([st.alpha, st.delta, st.kl_dist, st.surr_before, st.surr_after, st.vpg_dot_npg,
+                                   st.backtracks, st.cg_iters_run], np.float64)}
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes of outputs exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ======================================================================================= GPU arm
@@ -454,6 +484,8 @@ def run_gpu(args, cfg, rank, world, local_rank):
     wall = time.time() - t_wall
     launches = eng.kernel_launches() - launches0
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, stats[-1])
     ms = max_over_ranks(ms)
     ms_per_step = ms / args.steps
     fvp_ms_kernel = float(np.mean([s.fvp_kernel_ms_sum / max(1, s.fvp_launches) for s in stats]))
@@ -481,7 +513,7 @@ def run_gpu(args, cfg, rank, world, local_rank):
         agent.update_from_paths(fresh, GAMMA, LAM)
 
     e2e_warm = max(1, min(args.warmup, 3))
-    e2e_steps = max(1, min(args.steps, 10))
+    e2e_steps = args.steps
     for _ in range(e2e_warm):
         e2e_step()
     barrier()
@@ -626,7 +658,13 @@ def main():
     ap.add_argument("--no-hbm-roofline", action="store_true", help="skip the cfg5 linear-policy FVP measurement")
     ap.add_argument("--reference-sample-only", action="store_true",
                     help="--impl reference: skip the full-batch step (bounded sample + extrapolation only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the arrays the last timed step computed to DIR/<name>.npy (GPU arm, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm")
     cfg = CONFIGS[args.config]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -21,6 +21,21 @@ def load_golden(name):
     return g
 
 
+def golden_equal(a, g, key):
+    """`a` equals, bit for bit, the array a fixture stores under `key`: whole, or for a large array (stored by
+    oracle/make_golden_host.py's `exact`) its shape, its entries at the seeded sample positions and the sha256 of its
+    bytes."""
+    import hashlib
+    a = np.ascontiguousarray(a)
+    if key in g:
+        return np.array_equal(a, g[key])
+    sample = g[key + "@sample"]
+    if a.shape != tuple(g[key + "@shape"]) or a.dtype != sample.dtype:
+        return False
+    idx = np.sort(np.random.RandomState(0).choice(a.size, sample.size, replace=False))
+    return np.array_equal(a.ravel()[idx], sample) and hashlib.sha256(a.tobytes()).hexdigest() == str(g[key + "@sha256"])
+
+
 def golden_paths(g, demo=False):
     """Regenerate the synthetic trajectories a golden file was produced from and verify the checksum."""
     from oracle import npg_oracle as O

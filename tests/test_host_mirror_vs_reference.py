@@ -1,5 +1,6 @@
-"""The host-side policy containers (mjrl_b200.policies / utils.fc_network) against the live reference classes, on the CPU.
-Skipped where no reference checkout exists (the GPU box); there tests/test_agents_gpu.py exercises the same objects."""
+"""The host-side policy containers (mjrl_b200.policies / utils.fc_network) against the reference classes, on the CPU.
+The reference's outputs are stored in tests/golden/host_containers.npz (oracle/make_golden_host.py); the inputs are
+drawn here from the same seeded generators, in the same order."""
 import pickle
 import types
 
@@ -7,55 +8,53 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import ref_shim
-
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="needs the mjrl reference checkout")
+from conftest import golden_equal, load_golden
 
 
-def _pair(obs_dim, act_dim, hidden, seed, **kw):
-    R = ref_shim.load()
+@pytest.fixture(scope="module")
+def ref():
+    return load_golden("host_containers")
+
+
+SHAPES = [(6, 2, (32, 32)), (17, 6, (128, 128)), (5, 3, (64, 64))]      # mlp0_ .. mlp2_ in the fixture
+
+
+@pytest.mark.parametrize("shape", SHAPES)
+def test_policy_container_matches_reference(ref, shape):
     from mjrl_b200.policies.gaussian_mlp import MLP
-    spec = types.SimpleNamespace(observation_dim=obs_dim, action_dim=act_dim)
-    return R.MLP(R.EnvSpec(obs_dim, act_dim, 10), hidden_sizes=hidden, seed=seed, **kw), MLP(spec, hidden_sizes=hidden, seed=seed, **kw)
-
-
-@pytest.mark.parametrize("shape", [(6, 2, (32, 32)), (17, 6, (128, 128)), (5, 3, (64, 64))])
-def test_policy_container_matches_reference(shape):
     obs_dim, act_dim, hidden = shape
-    ref, mine = _pair(obs_dim, act_dim, hidden, seed=7, init_log_std=-0.25, min_log_std=-2.0)
-    assert mine.d == ref.d and [tuple(s) for s in mine.param_shapes] == [tuple(s) for s in ref.param_shapes]
-    assert list(mine.param_sizes) == list(ref.param_sizes)
-    assert np.array_equal(mine.get_param_values(), ref.get_param_values())          # same init draws, same layout
+    i = SHAPES.index(shape)
+    r = {k[len("mlp%d_" % i):]: v for k, v in ref.items() if k.startswith("mlp%d_" % i)}
+    mine = MLP(types.SimpleNamespace(observation_dim=obs_dim, action_dim=act_dim), hidden_sizes=hidden, seed=7,
+               init_log_std=-0.25, min_log_std=-2.0)
+    assert mine.d == r["d"] and repr([tuple(s) for s in mine.param_shapes]) == str(r["param_shapes"])
+    assert list(mine.param_sizes) == list(r["param_sizes"])
+    assert golden_equal(mine.get_param_values(), r, "init")                        # same init draws, same layout
     # set_param_values: layout, clamp of log_std, new / old sets
     rng = np.random.RandomState(1)
-    th = rng.randn(ref.d).astype(np.float32)
+    th = rng.randn(mine.d).astype(np.float32)
     th[-act_dim:] = np.linspace(-4.0, 1.0, act_dim)                                   # some entries below min_log_std
-    for flags in ((True, True), (True, False), (False, True)):
-        ref.set_param_values(th * (1 + flags[0] + 2 * flags[1]), *flags)
+    for j, flags in enumerate(((True, True), (True, False), (False, True))):
         mine.set_param_values(th * (1 + flags[0] + 2 * flags[1]), *flags)
-        assert np.array_equal(mine.get_param_values(), ref.get_param_values())
-        old_r = np.concatenate([p.data.numpy().ravel() for p in ref.old_params])
+        assert golden_equal(mine.get_param_values(), r, "set%d_params" % j)
         old_m = np.concatenate([p.data.numpy().ravel() for p in mine.old_params])
-        assert np.array_equal(old_m, old_r)
-        assert np.array_equal(mine.log_std_val, ref.log_std_val)
+        assert golden_equal(old_m, r, "set%d_old" % j)
+        assert golden_equal(mine.log_std_val, r, "set%d_log_std_val" % j)
     assert mine.get_param_values()[-act_dim:].min() >= -2.0
     # sampling: same mean, same global-RNG draw
     o = rng.randn(obs_dim)
-    np.random.seed(5); a_r, info_r = ref.get_action(o)
     np.random.seed(5); a_m, info_m = mine.get_action(o)
-    assert np.array_equal(a_m, a_r) and np.array_equal(info_m["mean"], info_r["mean"])
-    assert np.array_equal(info_m["evaluation"], info_r["evaluation"]) and np.array_equal(info_m["log_std"], info_r["log_std"])
+    assert golden_equal(a_m, r, "action") and golden_equal(info_m["mean"], r, "action_mean")
+    assert golden_equal(info_m["evaluation"], r, "action_evaluation") and golden_equal(info_m["log_std"], r, "action_log_std")
     # small-input helpers
     obs, act = rng.randn(50, obs_dim).astype(np.float32), rng.randn(50, act_dim).astype(np.float32)
-    mine.set_param_values(th, True, False); ref.set_param_values(th, True, False)     # new != old
-    np.testing.assert_allclose(mine.log_likelihood(obs, act), ref.log_likelihood(obs, act), rtol=1e-6, atol=1e-6)
-    nr, orr = ref.new_dist_info(obs, act), ref.old_dist_info(obs, act)
+    mine.set_param_values(th, True, False)                                            # new != old
+    np.testing.assert_allclose(mine.log_likelihood(obs, act), r["log_likelihood"], rtol=1e-6, atol=1e-6)
     nm, om = mine.new_dist_info(obs, act), mine.old_dist_info(obs, act)
-    for a, b in zip(nm[:2] + om[:2], nr[:2] + orr[:2]):
-        np.testing.assert_allclose(a.detach().numpy(), b.detach().numpy(), rtol=1e-6, atol=1e-6)
-    np.testing.assert_allclose(mine.likelihood_ratio(nm, om).detach().numpy(), ref.likelihood_ratio(nr, orr).detach().numpy(),
-                               rtol=1e-5, atol=1e-6)
-    np.testing.assert_allclose(float(mine.mean_kl(nm, om)), float(ref.mean_kl(nr, orr)), rtol=1e-5, atol=1e-7)
+    for a, b in zip(nm[:2] + om[:2], (r["new_ll"], r["new_mean"], r["old_ll"], r["old_mean"])):
+        np.testing.assert_allclose(a.detach().numpy(), b, rtol=1e-6, atol=1e-6)
+    np.testing.assert_allclose(mine.likelihood_ratio(nm, om).detach().numpy(), r["likelihood_ratio"], rtol=1e-5, atol=1e-6)
+    np.testing.assert_allclose(float(mine.mean_kl(nm, om)), float(r["mean_kl"]), rtol=1e-5, atol=1e-7)
     # pickling keeps the weights and keeps working
     clone = pickle.loads(pickle.dumps(mine))
     assert np.array_equal(clone.get_param_values(), mine.get_param_values())
@@ -63,34 +62,29 @@ def test_policy_container_matches_reference(shape):
     assert np.array_equal(clone.get_param_values()[:-act_dim], (th * 0.5)[:-act_dim])
 
 
-def test_fc_network_matches_reference():
-    ref_shim.load()
-    from mjrl.utils.fc_network import FCNetwork as RefNet
+def test_fc_network_matches_reference(ref):
     from mjrl_b200.utils.fc_network import FCNetwork
     rng = np.random.RandomState(0)
     tr = dict(in_shift=rng.randn(7), in_scale=0.5 + rng.rand(7), out_shift=rng.randn(3), out_scale=0.5 + rng.rand(3))
-    for hidden, nl in (((16, 8), "tanh"), ((32, 32), "relu"), ((), "tanh")):
-        torch.manual_seed(3); a = RefNet(7, 3, hidden, nl, **tr)
+    for i, (hidden, nl) in enumerate((((16, 8), "tanh"), ((32, 32), "relu"), ((), "tanh"))):
+        k = "fc%d_" % i
         torch.manual_seed(3); b = FCNetwork(7, 3, hidden, nl, **tr)
-        assert [tuple(p.shape) for p in a.parameters()] == [tuple(p.shape) for p in b.parameters()]
-        assert all(torch.equal(p, q) for p, q in zip(a.parameters(), b.parameters()))
-        assert list(a.state_dict().keys()) == list(b.state_dict().keys())
+        assert repr([tuple(p.shape) for p in b.parameters()]) == str(ref[k + "param_shapes"])
+        assert golden_equal(np.concatenate([p.data.numpy().ravel() for p in b.parameters()]), ref, k + "params")
+        assert repr(list(b.state_dict().keys())) == str(ref[k + "state_dict_keys"])
         x = torch.from_numpy(rng.randn(9, 7).astype(np.float32))
-        assert torch.equal(a(x), b(x))
-        assert b.layer_sizes == a.layer_sizes and set(b.transformations) == set(a.transformations)
+        assert golden_equal(b(x).detach().numpy(), ref, k + "output")
+        assert repr(b.layer_sizes) == str(ref[k + "layer_sizes"])
+        assert repr(sorted(b.transformations)) == str(ref[k + "transformations"])
 
 
-def test_linear_policy_container_matches_reference():
-    R = ref_shim.load()
+def test_linear_policy_container_matches_reference(ref):
     from mjrl_b200.policies.gaussian_linear import LinearPolicy
-    spec = types.SimpleNamespace(observation_dim=11, action_dim=4)
-    ref = R.LinearPolicy(R.EnvSpec(11, 4, 10), seed=3)
-    mine = LinearPolicy(spec, seed=3)
-    assert mine.d == ref.d
-    th = np.random.RandomState(2).randn(ref.d).astype(np.float32)
-    ref.set_param_values(th); mine.set_param_values(th)
-    assert np.array_equal(mine.get_param_values(), ref.get_param_values())
+    mine = LinearPolicy(types.SimpleNamespace(observation_dim=11, action_dim=4), seed=3)
+    assert mine.d == ref["lin_d"]
+    th = np.random.RandomState(2).randn(mine.d).astype(np.float32)
+    mine.set_param_values(th)
+    assert golden_equal(mine.get_param_values(), ref, "lin_params")
     o = np.random.RandomState(4).randn(11)
-    np.random.seed(9); a_r = ref.get_action(o)[0]
     np.random.seed(9); a_m = mine.get_action(o)[0]
-    np.testing.assert_allclose(a_m, a_r, rtol=1e-6, atol=1e-6)
+    np.testing.assert_allclose(a_m, ref["lin_action"], rtol=1e-6, atol=1e-6)

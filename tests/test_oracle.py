@@ -1,16 +1,13 @@
 """CPU tests: the oracle restatement (oracle/npg_oracle.py) against (a) known-answer vectors and
-(b) the golden fixtures produced by the real reference (oracle/make_golden.py), and (c) the live
-reference when a checkout is present.  Tolerances: bit-exact for returns/GAE/indexing; fp32
+(b) the golden fixtures produced by the real reference (oracle/make_golden.py), and (c) one reference
+NPG step on shapes of its own (oracle/make_golden_host.py).  Tolerances: bit-exact for returns/GAE/indexing; fp32
 autograd flavour == reference to ~1e-6; fp64 closed form == reference to fp32 rounding."""
-import copy
-
 import numpy as np
 import pytest
 import torch
 
-from conftest import ALL_CASES, golden_paths, load_golden, one_minus_cos, rel
+from conftest import ALL_CASES, golden_equal, golden_paths, load_golden, one_minus_cos, rel
 from oracle import npg_oracle as O
-from oracle import ref_shim
 
 
 def spec_of(g):
@@ -165,32 +162,23 @@ def test_fit_needs_two_batches():
         O.vf_fit(O.VFState(3), paths, [np.arange(100)])
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="needs the mjrl reference checkout")
 def test_live_reference_npg_step():
-    """Fresh shapes not in the goldens: oracle (fp32 autograd flavour) vs the reference run here."""
-    R = ref_shim.load()
+    """Shapes not in the other goldens: oracle (fp32 autograd flavour) vs one NPG step of the reference, whose
+    initial weights, returns, advantages and new parameters are stored in tests/golden/npg_11x3_ragged.npz."""
+    g = load_golden("npg_11x3_ragged")
     torch.set_num_threads(1)
     obs_dim, act_dim, hidden = 11, 3, (64, 64)
     paths = O.synthetic_paths(obs_dim, act_dim, 30, 300, seed=3, ragged=True)
-    es = R.EnvSpec(obs_dim, act_dim, 300)
-    pol = R.MLP(es, hidden_sizes=hidden, seed=9)
-    bl = R.MLPBaseline(es, reg_coef=1e-3, epochs=1)
     spec = O.PolicySpec(obs_dim, act_dim, hidden)
-    th = pol.get_param_values()
+    th = g["theta0"]
     vf = O.VFState(obs_dim)
-    vf.w = np.concatenate([p.data.numpy().ravel() for p in bl.model.parameters()])
-    ref_paths, or_paths = copy.deepcopy(paths), copy.deepcopy(paths)
-    R.process_samples.compute_returns(ref_paths, 0.995)
-    R.process_samples.compute_advantages(ref_paths, bl, 0.995, 0.97)
-    O.compute_returns(or_paths, 0.995)
-    O.compute_advantages(or_paths, lambda p: O.vf_predict(vf, p), 0.995, 0.97)
-    for a, b in zip(ref_paths, or_paths):
-        assert np.array_equal(a["returns"], b["returns"])
-        assert np.array_equal(a["advantages"], b["advantages"])
-    agent = R.NPG(None, pol, bl, normalized_step_size=0.05)
-    agent.train_from_paths(ref_paths)
+    vf.w = g["vf_w"].copy()
+    O.compute_returns(paths, 0.995)
+    O.compute_advantages(paths, lambda p: O.vf_predict(vf, p), 0.995, 0.97)
+    assert golden_equal(np.concatenate([p["returns"] for p in paths]), g, "returns")
+    assert golden_equal(np.concatenate([p["advantages"] for p in paths]), g, "advantages")
     obs = np.concatenate([p["observations"] for p in paths])
     act = np.concatenate([p["actions"] for p in paths])
-    adv = O.whiten(np.concatenate([p["advantages"] for p in or_paths]))
+    adv = O.whiten(np.concatenate([p["advantages"] for p in paths]))
     o = O.policy_update(spec, th, obs, act, adv, "npg", step_size=0.05)
-    assert rel(o["new_params"], pol.get_param_values()) < 1e-4
+    assert rel(o["new_params"], g["new_params"]) < 1e-4
