@@ -17,8 +17,8 @@
 // The B operand's two terms are N-concatenated ([B hi | B lo] are adjacent column groups), so a product costs two
 // MMAs per k-step; small operands carry power-of-two scales (SW, SA, SG below) that keep their fp16 low terms normal.
 // State: W2's fp32 master copy lives in registers (32 per thread), its Adam moments in TMEM (2 x 128 columns), W1's
-// state and the small vectors in shared memory.  512 threads; thread 0 issues the MMAs; gW2 is issued before dh1 so
-// that half of W2's Adam update runs under the dh1 GEMM.
+// state and the small vectors in shared memory.  512 threads; one elected lane of a converged warp 0 issues the MMAs;
+// gW2 is issued before dh1 so that half of W2's Adam update runs under the dh1 GEMM.
 // Semantics (minibatch order, 1/B scaling, L2-in-gradient weight decay, bias correction, state persistence) are the
 // reference's; sums run in a fixed order (deterministic).
 #include <cuda_fp16.h>
@@ -353,6 +353,15 @@ __device__ __forceinline__ void ks_helper(const TcFitArgs& a, unsigned char* sme
     if (warp == 0) tmem_dealloc(tmem, HT_COLS);
 }
 
+// one lane of a converged warp: the MMA issuer.  Warp 0 enters the issue block whole and elect.sync picks the lane, so
+// the issue loop runs converged instead of in a divergent tid == 0 branch (52 instead of 62 cycles per N = 64 MMA in
+// tools/mma_rate_probe.cu)
+__device__ __forceinline__ bool elect_one() {
+    uint32_t p;
+    asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}\n" : "=r"(p));
+    return p != 0;
+}
+
 // PROF = true instantiates the per-phase clock64 counters (tools/vf_fit_profile.py); the production instance carries none
 // of that code.  Code size matters here: a single resident CTA runs a ~2.7 k-instruction step body 15 624 times, and a
 // body that does not fit the 32 KB instruction cache is re-fetched from L2 every step (the fetch stalls showed up as
@@ -490,12 +499,15 @@ __global__ void __launch_bounds__(NT, 1) vf_fit_tc_kernel(const TcFitArgs a) {
     for (int s = 0; s < a.steps; ++s) {
         sync_ops();                                                  // X(s), weights(s) staged
         TC_PROF(13);                                                 // (barrier skew at the top of the step)
-        if (tid == 0) {                                              // layer 1: z1^T = W1 x^T
+        if (warp == 0) {                                             // layer 1: z1^T = W1 x^T
             tcgen05_fence_after();
-            const uint32_t xb = sbase + ((s & 1) ? S_X2 : S_XH);
-            gemm3<KP / 16>(tmem + T_D, sbase + S_W1H, sbase + S_W1L, 2 * LB128, LB128, 128,
-                           xb, xb + X_BYTES, 2 * LB64, LB64, 128, ID_L1);
-            mma_commit(&bars[0]);
+            if (elect_one()) {
+                const uint32_t xb = sbase + ((s & 1) ? S_X2 : S_XH);
+                gemm3<KP / 16>(tmem + T_D, sbase + S_W1H, sbase + S_W1L, 2 * LB128, LB128, 128,
+                               xb, xb + X_BYTES, 2 * LB64, LB64, 128, ID_L1);
+                mma_commit(&bars[0]);
+            }
+            __syncwarp();
         }
         TC_PROF(14);                                                 // (issue of the six layer-1 MMAs)
         const float4 cst = cst_next;
@@ -551,11 +563,14 @@ __global__ void __launch_bounds__(NT, 1) vf_fit_tc_kernel(const TcFitArgs a) {
         }
         sync_ops();
         TC_PROF(2);
-        if (tid == 0) {                                              // layer 2: z2^T = W2 h1
+        if (warp == 0) {                                             // layer 2: z2^T = W2 h1
             tcgen05_fence_after();
-            gemm2c<H / 16>(tmem + T_D, sbase + S_W2H, sbase + S_W2L, 2 * LB128, LB128, 128,
-                           sbase + S_HH, 2 * 128, 128, LB128, ID_L2c, ID_L2);
-            mma_commit(&bars[0]);
+            if (elect_one()) {
+                gemm2c<H / 16>(tmem + T_D, sbase + S_W2H, sbase + S_W2L, 2 * LB128, LB128, 128,
+                               sbase + S_HH, 2 * 128, 128, LB128, ID_L2c, ID_L2);
+                mma_commit(&bars[0]);
+            }
+            __syncwarp();
         }
         TC_PROF(3);
         // gathers for the coming steps, issued while the layer-2 GEMM runs and nobody has work: rows of step s+1 (consumed
@@ -641,14 +656,17 @@ __global__ void __launch_bounds__(NT, 1) vf_fit_tc_kernel(const TcFitArgs a) {
         }
         sync_ops();
         TC_PROF(6);
-        if (tid == 0) {                                              // gW2 = dz2 h1^T -> bar 1, then dh1^T = W2^T dz2 -> bar 0
+        if (warp == 0) {                                             // gW2 = dz2 h1^T -> bar 1, then dh1^T = W2^T dz2 -> bar 0
             tcgen05_fence_after();
-            gemm3<NB / 16>(tmem + T_G2, sbase + S_DH, sbase + S_DL, 2 * LB128, LB128, 128,
-                           sbase + S_HH, sbase + S_HL, 2 * LB128, LB128, 128, ID_G2);
-            mma_commit(&bars[1]);
-            gemm2c<H / 16>(tmem + T_D, sbase + S_W2H, sbase + S_W2L, 2 * 128, 128, LB128,
-                           sbase + S_DH, 2 * 128, 128, LB128, ID_DHc, ID_DH);
-            mma_commit(&bars[0]);
+            if (elect_one()) {
+                gemm3<NB / 16>(tmem + T_G2, sbase + S_DH, sbase + S_DL, 2 * LB128, LB128, 128,
+                               sbase + S_HH, sbase + S_HL, 2 * LB128, LB128, 128, ID_G2);
+                mma_commit(&bars[1]);
+                gemm2c<H / 16>(tmem + T_D, sbase + S_W2H, sbase + S_W2L, 2 * 128, 128, LB128,
+                               sbase + S_DH, 2 * 128, 128, LB128, ID_DHc, ID_DH);
+                mma_commit(&bars[0]);
+            }
+            __syncwarp();
         }
         TC_PROF(7);
         // ---- nothing depends on these until the next step: they run while the gW2 GEMM has the tensor pipe to itself ----
@@ -728,11 +746,14 @@ __global__ void __launch_bounds__(NT, 1) vf_fit_tc_kernel(const TcFitArgs a) {
         sync_ops();
         TC_PROF(9);
         if (KS && tid == 0) flag_release(a.flags, s + 1);            // every thread's dz1 rows are written (barrier above)
-        if (tid == 0) {                                              // gW1 = dz1 x -> bar 0, under the second Adam half of W2
+        if (warp == 0) {                                             // gW1 = dz1 x -> bar 0, under the second Adam half of W2
             tcgen05_fence_after();
-            gemm2c<NB / 16>(tmem + T_G1, sbase + S_DH, sbase + S_DL, 2 * LB128, LB128, 128,
-                            sbase + ((s & 1) ? S_X2 : S_XH), 2 * 128, 128, LB64, ID_G1c, ID_G1);
-            mma_commit(&bars[0]);
+            if (elect_one()) {
+                gemm2c<NB / 16>(tmem + T_G1, sbase + S_DH, sbase + S_DL, 2 * LB128, LB128, 128,
+                                sbase + ((s & 1) ? S_X2 : S_XH), 2 * 128, 128, LB64, ID_G1c, ID_G1);
+                mma_commit(&bars[0]);
+            }
+            __syncwarp();
         }
         store_w2(0);
         adam_w2(1);
