@@ -164,6 +164,32 @@ int  mjb_policy_last_vectors(mjb_engine* e, float* vpg_out, float* npg_out);   /
  * row stride); n_each[i] <= n_idx says how many entries of row i are valid.  One-shot: consumed by that call. */
 int  mjb_policy_set_hvp_lengths(mjb_engine* e, const int64_t* n_each, int iters);
 
+/* ---- minibatch-Adam policy training: PPO-clip and behaviour cloning -------------------------- */
+/* loss_kind: MJB_LOSS_PPO = -mean(min(LR A, clip(LR, 1-clip_coef, 1+clip_coef) A)) with LR = exp(LL - LL_old) on the whitened
+ * advantages of mjb_process_paths and LL_old of the old parameters and transforms (algos/ppo_clip.py:48-55,88-97);
+ * MJB_LOSS_BC_MLE = -mean(LL), MJB_LOSS_BC_MSE = mean((mu - a)^2) on the resident batch's actions
+ * (algos/behavior_cloning.py:83-105,120-127).  Runs `steps` sequential torch.optim.Adam steps (lr, betas 0.9/0.999,
+ * eps 1e-8, no weight decay) on theta_new, one minibatch of `batch` (<= 64) resident rows per step, rows idx[step][0..batch)
+ * (host-or-device int32 [steps][batch]).  The whole chain is one kernel launch on one SM.  log_std is not clamped inside
+ * the chain (the reference clamps in set_param_values after it); MSE leaves log_std and its Adam moments untouched (it has
+ * no gradient, so torch's Adam skips it).  Afterwards mjb_policy_eval reports surr_after / kl_dist of the unclamped
+ * parameters.  loss_out / clip_frac_out (nullable, host-or-device, steps floats): every step's minibatch loss and the
+ * fraction of its rows whose gradient the PPO clip zeroed (0 for the BC losses).  Single GPU, MLP policy only. */
+enum { MJB_LOSS_PPO = 0, MJB_LOSS_BC_MLE = 1, MJB_LOSS_BC_MSE = 2 };
+int  mjb_policy_sgd(mjb_engine* e, int loss_kind, const int32_t* idx, int64_t steps, int batch, float lr, float clip_coef,
+                    float* loss_out, float* clip_frac_out);
+/* Adam state of the policy optimizer (torch.optim.Adam(policy.trainable_params), ppo_clip.py:46, behavior_cloning.py:42):
+ * moments in the flat theta layout (d floats each, host-or-device) and the step count; it lives on the device and
+ * persists across mjb_policy_sgd calls.  NULL / step < 0 leave that part unchanged. */
+int  mjb_policy_adam_set(mjb_engine* e, const float* m, const float* v, int64_t step);
+int  mjb_policy_adam_get(mjb_engine* e, float* m, float* v, int64_t* step);
+/* Full-batch BC loss of theta_new over the resident batch (behavior_cloning.py:115-118,132-135: loss_before / loss_after);
+ * loss_kind MJB_LOSS_BC_MLE or MJB_LOSS_BC_MSE.  Uses the old-policy cache buffers as scratch (the cache is rebuilt when
+ * next needed). */
+int  mjb_policy_bc_loss(mjb_engine* e, int loss_kind, double* out);
+/* CUDA-event time of the last mjb_policy_sgd kernel (the whole chain). */
+int  mjb_policy_sgd_timing(mjb_engine* e, float* last_ms);
+
 /* FVP arithmetic: 1 (default where supported: 128x128 MLP, obs < 32, act <= 8) = tcgen05 tensor cores with two-term
  * fp16 operand splitting (hi*hi + lo*hi + hi*lo, fp32 accumulation in TMEM); 0 = the fp32 FMA tile kernel.
  * Returns 1 (not an error) when tensor cores were requested for a shape that only has the FMA kernel. */

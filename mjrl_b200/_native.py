@@ -86,6 +86,11 @@ _SIGNATURES = {
     "mjb_policy_set_tensor_cores": (C.c_int, [_P, C.c_int]),
     "mjb_policy_last_vectors": (C.c_int, [_P, _P, _P]),
     "mjb_policy_set_hvp_lengths": (C.c_int, [_P, _P, C.c_int]),
+    "mjb_policy_sgd": (C.c_int, [_P, C.c_int, _P, C.c_int64, C.c_int, C.c_float, C.c_float, _P, _P]),
+    "mjb_policy_adam_set": (C.c_int, [_P, _P, _P, C.c_int64]),
+    "mjb_policy_adam_get": (C.c_int, [_P, _P, _P, C.POINTER(C.c_int64)]),
+    "mjb_policy_bc_loss": (C.c_int, [_P, C.c_int, C.POINTER(C.c_double)]),
+    "mjb_policy_sgd_timing": (C.c_int, [_P, C.POINTER(C.c_float)]),
     "mjb_vf_dim": (C.c_int, [_P]),
     "mjb_vf_set_state": (C.c_int, [_P, _P, _P, _P, C.c_int64]),
     "mjb_vf_get_state": (C.c_int, [_P, _P, _P, _P, C.POINTER(C.c_int64)]),

@@ -15,6 +15,9 @@ class BatchREINFORCE:
     `desired_kl` line search (batch_reinforce.py:117-176) is a first-order method outside the NPG path."""
 
     algo = "npg"
+    # Start the baseline fit before train_from_paths, on the engine's side stream.  Only valid when the reference draws
+    # nothing from numpy's global RNG inside train_from_paths before the fit's permutations (PPO does: its minibatches).
+    fit_overlap = True
 
     def _setup(self, env, policy, baseline, seed, save_logs):
         self.env, self.policy, self.baseline = env, policy, baseline
@@ -145,7 +148,7 @@ class BatchREINFORCE:
         # evaluated, then the fit permutations, A9); that order is only reproducible with the fit AFTER the policy
         # step, so the overlap is switched off for that setting.
         subsampling = getattr(self, "hvp_subsample", None) is not None and self.hvp_subsample < 0.99
-        overlap = hasattr(self.baseline, "fit_begin") and not subsampling
+        overlap = self.fit_overlap and hasattr(self.baseline, "fit_begin") and not subsampling
         process_samples.returns_on(eng, paths, gamma, write_back=not overlap)
         error_before = error_after = None
         fit_started = False

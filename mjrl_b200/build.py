@@ -12,7 +12,8 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "build")
 LIB = os.path.join(HERE, "libmjrl_b200.so")
 SOURCES = ["engine.cu", "mlp_h32.cu", "mlp_h64.cu", "mlp_h128.cu", "mlp_h256.cu", "linear_kernel.cu",
-           "scan.cu", "vecops.cu", "vf_fit.cu", "fvp_tc.cu", "linear_tc.cu", "vf_fit_tc.cu", "host_perm.cu", "p2p.cu", "ridge.cu"]
+           "scan.cu", "vecops.cu", "vf_fit.cu", "fvp_tc.cu", "linear_tc.cu", "vf_fit_tc.cu", "host_perm.cu", "p2p.cu", "ridge.cu",
+           "policy_sgd.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O2"]
 

@@ -152,6 +152,13 @@ struct mjb_engine {
     const CgGraph* last_cg_graph = nullptr;       // set when the last CG ran as a graph (its events time the FVP launches)
     cudaEvent_t fit_ev[2] = {nullptr, nullptr};     // around the sequential Adam kernels of the last fit (on its stream)
     bool fit_timed = false;
+    // ---- minibatch-Adam policy training (policy_sgd.cu): Adam moments / step count, index block, per-step outputs
+    float *sgd_m = nullptr, *sgd_v = nullptr, *sgd_wT = nullptr;
+    long long sgd_step = 0;
+    int* sgd_idx = nullptr; long long sgd_idx_cap = 0;
+    float* sgd_out = nullptr; long long sgd_out_cap = 0;  // [2][cap]: per-step loss, clip fraction
+    cudaEvent_t sgd_ev[2] = {nullptr, nullptr};     // around the last policy_sgd kernel
+    bool sgd_timed = false;
 };
 
 enum {  // slots in dsc
@@ -167,6 +174,7 @@ enum {  // slots in dsc
     DS_RET = 20,       // path-return stats: sum, sumsq, min, max, n
     DS_VF = 26,        // vf error sums (2)
     DS_TCSCALE = 28,   // FVP scale with the tangent's power-of-two pre-scale undone (2)
+    DS_BCLOSS = 30,    // full-batch behaviour-cloning loss sum
     DS_TOTAL = 32
 };
 
@@ -551,7 +559,8 @@ void mjb_destroy(mjb_engine* e) {
                     e->prep_tan, e->tc_prep_new, e->tc_prep_tan, e->tc_vscale, e->obs, e->act, e->rew, e->path_off, e->term, e->tstep, e->ret, e->adv, e->base,
                     e->adv_white, e->weights, e->path_ret, e->ll_old, e->mu_old, e->gpartial, e->eval_partial,
                     e->mom_scratch, e->dsc, e->g, e->x, e->r, e->p, e->Fp, e->tmpv, e->idx_dev, e->stage64, e->vf_w,
-                    e->vf_m, e->vf_v, e->vf_wT, e->vf_prep, e->vf_feat, e->vf_ret32, e->vf_consts, e->vf_ks, e->perm_dev, e->fit_obs, e->fit_tstep, e->fit_ret};
+                    e->vf_m, e->vf_v, e->vf_wT, e->vf_prep, e->vf_feat, e->vf_ret32, e->vf_consts, e->vf_ks, e->perm_dev, e->fit_obs, e->fit_tstep, e->fit_ret,
+                    e->sgd_m, e->sgd_v, e->sgd_wT, e->sgd_idx, e->sgd_out};
     for (void* b : bufs) if (b) cudaFree(b);
     if (e->pinned) cudaFreeHost(e->pinned);
     if (e->h_dsc) cudaFreeHost(e->h_dsc);
@@ -559,6 +568,7 @@ void mjb_destroy(mjb_engine* e) {
     for (auto& ev : e->user_ev) if (ev) cudaEventDestroy(ev);
     for (auto& pr : e->fvp_ev) for (auto& ev : pr) if (ev) cudaEventDestroy(ev);
     for (auto& ev : e->fit_ev) if (ev) cudaEventDestroy(ev);
+    for (auto& ev : e->sgd_ev) if (ev) cudaEventDestroy(ev);
     if (e->stream_vf) { cudaStreamSynchronize(e->stream_vf); cudaStreamDestroy(e->stream_vf); }
     if (e->stream) cudaStreamDestroy(e->stream);
     delete e;
@@ -591,6 +601,7 @@ int mjb_create(const mjb_config* cfg, mjb_engine** out) {
     for (auto& ev : e->user_ev) if (cudaEventCreate(&ev) != cudaSuccess) return fail("event create failed");
     for (auto& pr : e->fvp_ev) for (auto& ev : pr) if (cudaEventCreate(&ev) != cudaSuccess) return fail("event create failed");
     for (auto& ev : e->fit_ev) if (cudaEventCreate(&ev) != cudaSuccess) return fail("event create failed");
+    for (auto& ev : e->sgd_ev) if (cudaEventCreate(&ev) != cudaSuccess) return fail("event create failed");
 
     e->linear = cfg->n_hidden == 0;
     e->A = cfg->act_dim;
@@ -649,6 +660,8 @@ int mjb_create(const mjb_config* cfg, mjb_engine** out) {
     ALLOC(e->vf_w, e->vf_d); ALLOC(e->vf_m, e->vf_d); ALLOC(e->vf_v, e->vf_d);
     ALLOC(e->vf_wT, (size_t)(O + 4) * vh0 + (size_t)vh0 * vh1);
     ALLOC(e->vf_prep, e->VPL.total);
+    ALLOC(e->sgd_m, e->d); ALLOC(e->sgd_v, e->d);
+    if (!e->linear) ALLOC(e->sgd_wT, policy_sgd_scratch_floats(cfg->obs_dim, cfg->hidden[0], cfg->hidden[1], cfg->act_dim));
 #undef ALLOC
     e->pinned_bytes = std::min<size_t>(N * std::max(O, A) * sizeof(double), (size_t)64 << 20);
     e->pinned_bytes = std::max<size_t>(e->pinned_bytes, (size_t)1 << 20);
@@ -1307,6 +1320,108 @@ int mjb_policy_step(mjb_engine* e, int algo, double step_size_or_kl, double cons
         e->last_fvp_ms = ms;
     }
     if (out) *out = st;
+    return 0;
+}
+
+// ------------------------------------------------------------------------ minibatch-Adam policy training
+int mjb_policy_sgd(mjb_engine* e, int loss_kind, const int32_t* idx, int64_t steps, int batch, float lr, float clip_coef,
+                   float* loss_out, float* clip_frac_out) {
+    if (e->cfg.world_size > 1) FAIL(e, "mjb_policy_sgd: single-GPU only (the chain is not replicated across ranks)");
+    if (e->linear) FAIL(e, "mjb_policy_sgd: the minibatch-Adam kernel covers the Gaussian MLP policy, not LinearPolicy");
+    if (loss_kind != SGD_PPO && loss_kind != SGD_BC_MLE && loss_kind != SGD_BC_MSE) FAIL(e, "mjb_policy_sgd: bad loss kind");
+    if (batch < 1 || batch > 64) FAIL(e, "mjb_policy_sgd: minibatch size must be in [1, 64]");
+    if (steps < 0 || steps > 0x7fffffffLL) FAIL(e, "mjb_policy_sgd: bad step count");
+    if (policy_sgd_smem_bytes(e->cfg.obs_dim, e->cfg.hidden[0], e->cfg.hidden[1], e->A) > policy_sgd_max_smem())
+        FAIL(e, "mjb_policy_sgd: obs_dim too large for the kernel's shared-memory activations at this width");
+    if (e->n_roll <= 0) FAIL(e, "mjb_policy_sgd: no batch resident");
+    if (loss_kind == SGD_PPO && !e->have_white) FAIL(e, "mjb_policy_sgd: PPO needs mjb_process_paths first");
+    if (steps == 0) return 0;
+    if (loss_kind == SGD_PPO && ensure_old_cache(e, e->n_roll)) return -1;    // LL under the old policy and transforms
+    const long long total = steps * (long long)batch;
+    if (total > e->sgd_idx_cap) {
+        if (e->sgd_idx) cudaFree(e->sgd_idx);
+        e->sgd_idx = nullptr; e->sgd_idx_cap = 0;
+        CK(e, cudaMalloc(&e->sgd_idx, sizeof(int) * total));
+        e->sgd_idx_cap = total;
+    }
+    if (copy_in(e, e->sgd_idx, idx, sizeof(int) * total)) return -1;
+    if ((loss_out || clip_frac_out) && steps > e->sgd_out_cap) {
+        if (e->sgd_out) cudaFree(e->sgd_out);
+        e->sgd_out = nullptr; e->sgd_out_cap = 0;
+        CK(e, cudaMalloc(&e->sgd_out, sizeof(float) * 2 * steps));
+        e->sgd_out_cap = steps;
+    }
+    PolicySgdArgs a;
+    a.K0 = e->cfg.obs_dim; a.h1 = e->cfg.hidden[0]; a.h2 = e->cfg.hidden[1]; a.A = e->A; a.loss_kind = loss_kind;
+    a.obs = e->obs; a.act = e->act; a.adv = e->adv_white; a.ll_old = e->ll_old;
+    a.in_shift = e->pnew.in_shift; a.in_scale = e->pnew.in_scale; a.out_shift = e->pnew.out_shift; a.out_scale = e->pnew.out_scale;
+    a.idx = e->sgd_idx; a.steps = steps; a.batch = batch;
+    a.lr = lr; a.beta1 = 0.9f; a.beta2 = 0.999f; a.eps = 1e-8f;
+    a.clip_lo = (float)(1.0 - (double)clip_coef); a.clip_hi = (float)(1.0 + (double)clip_coef);
+    a.step0 = e->sgd_step;
+    a.theta = e->pnew.theta; a.m = e->sgd_m; a.v = e->sgd_v; a.wT = e->sgd_wT;
+    a.loss_out = loss_out ? e->sgd_out : nullptr;
+    a.clip_out = clip_frac_out ? e->sgd_out + steps : nullptr;     // (all zero for the BC losses)
+    CK(e, cudaEventRecord(e->sgd_ev[0], e->stream));
+    const cudaError_t ce = launch_policy_sgd(a, e->stream);
+    if (ce != cudaSuccess) FAIL(e, std::string("policy_sgd launch: ") + cudaGetErrorString(ce));
+    CK(e, cudaEventRecord(e->sgd_ev[1], e->stream));
+    e->launches += 1;
+    e->sgd_timed = true;
+    e->sgd_step += steps;
+    // theta_new changed in place: refresh what is keyed on it (no log_std clamp here -- the reference evaluates
+    // surr_after / kl_dist before set_param_values clamps, ppo_clip.py:99-102)
+    launch_prep_mlp(e->pnew.theta, e->PL, e->pnew.prep, e->stream);
+    e->launches += 1;
+    if (e->tc_ok) { launch_tc_prep(e->pnew.theta, e->PL, nullptr, e->tc_prep_new, e->stream); e->launches += 1; }
+    e->old_equals_new = false;
+    CK(e, cudaGetLastError());
+    if (loss_out) CK(e, cudaMemcpyAsync(loss_out, e->sgd_out, sizeof(float) * steps, cudaMemcpyDefault, e->stream));
+    if (clip_frac_out) CK(e, cudaMemcpyAsync(clip_frac_out, a.clip_out, sizeof(float) * steps, cudaMemcpyDefault, e->stream));
+    CK(e, cudaStreamSynchronize(e->stream));
+    return 0;
+}
+
+int mjb_policy_adam_set(mjb_engine* e, const float* m, const float* v, int64_t step) {
+    if (m && copy_in(e, e->sgd_m, m, sizeof(float) * e->d)) return -1;
+    if (v && copy_in(e, e->sgd_v, v, sizeof(float) * e->d)) return -1;
+    if (step >= 0) e->sgd_step = step;
+    CK(e, cudaStreamSynchronize(e->stream));
+    return 0;
+}
+
+int mjb_policy_adam_get(mjb_engine* e, float* m, float* v, int64_t* step) {
+    if (m && d2any(e, m, e->sgd_m, sizeof(float) * e->d)) return -1;
+    if (v && d2any(e, v, e->sgd_v, sizeof(float) * e->d)) return -1;
+    if (step) *step = e->sgd_step;
+    return 0;
+}
+
+int mjb_policy_bc_loss(mjb_engine* e, int loss_kind, double* out) {
+    if (loss_kind != SGD_BC_MLE && loss_kind != SGD_BC_MSE) FAIL(e, "mjb_policy_bc_loss: loss kind must be MLE or MSE");
+    if (e->cfg.world_size > 1) FAIL(e, "mjb_policy_bc_loss: single-GPU only");
+    if (e->n_roll <= 0) FAIL(e, "mjb_policy_bc_loss: no batch resident");
+    // the EVAL tile kernel writes per-row LL / mean of theta_new into the old-policy cache buffers: the cache is void after
+    const int grid = run_policy(e, MODE_EVAL, e->pnew, nullptr, e->n_roll, nullptr, nullptr, OLD_WRITE);
+    if (grid < 0) return -1;
+    e->old_cache_valid = false;
+    if (launch_bc_loss_sum(e->ll_old, e->mu_old, e->act, e->n_roll, e->A, loss_kind, e->mom_scratch, e->dsc + DS_BCLOSS,
+                           e->stream) != cudaSuccess) FAIL(e, "bc loss launch failed");
+    e->launches += 2;
+    CK(e, cudaMemcpyAsync(e->h_dsc + DS_BCLOSS, e->dsc + DS_BCLOSS, sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    CK(e, cudaStreamSynchronize(e->stream));
+    const double sum = e->h_dsc[DS_BCLOSS];
+    // torch.mean in fp32: round the mean to fp32 like the reference's scalar
+    *out = loss_kind == SGD_BC_MLE ? (double)(float)(-sum / (double)e->n_roll)
+                                   : (double)(float)(sum / ((double)e->n_roll * (double)e->A));
+    return 0;
+}
+
+int mjb_policy_sgd_timing(mjb_engine* e, float* last_ms) {
+    *last_ms = 0.f;
+    if (!e->sgd_timed) return 0;
+    CK(e, cudaEventSynchronize(e->sgd_ev[1]));
+    CK(e, cudaEventElapsedTime(last_ms, e->sgd_ev[0], e->sgd_ev[1]));
     return 0;
 }
 

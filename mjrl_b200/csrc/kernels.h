@@ -161,4 +161,30 @@ cudaError_t launch_vf_fit_tc(const VfFitArgs& a, const float* feat, const float*
 // err = sum((ret - pred)^2) / (sum(ret^2) + 1e-8) pieces: out = {sum err^2, sum ret^2} (fp32 casts like the reference)
 void launch_vf_error(const double* ret, const float* pred, long long n, double* scratch, double* out2, cudaStream_t s);
 
+// ---- policy_sgd.cu : sequential minibatch Adam of the Gaussian-MLP policy (PPO-clip, behaviour cloning)
+enum { SGD_PPO = 0, SGD_BC_MLE = 1, SGD_BC_MSE = 2 };
+struct PolicySgdArgs {
+    int K0, h1, h2, A;                // real widths (K0 = obs_dim)
+    int loss_kind;                    // SGD_*
+    const float* obs; const float* act;            // resident batch rows
+    const float* adv; const float* ll_old;         // PPO: whitened advantages, log-likelihood under the old policy
+    const float* in_shift; const float* in_scale; const float* out_shift; const float* out_scale;
+    const int* idx;                   // [steps][batch] rows of every minibatch
+    long long steps; int batch;
+    float lr, beta1, beta2, eps;
+    float clip_lo, clip_hi;           // PPO: 1 - clip_coef, 1 + clip_coef
+    long long step0;                  // optimizer steps taken before this launch
+    float* theta; float* m; float* v; // flat reference layout, updated in place
+    float* wT;                        // scratch: W1T [K0][h1], W2T [h1][h2], new W3 / b3 [A (h2 + 1)]
+    float* loss_out;                  // [steps] minibatch loss (optional)
+    float* clip_out;                  // [steps] fraction of rows whose gradient the clip zeroed (optional, PPO)
+};
+inline size_t policy_sgd_max_smem() { return 226 * 1024; }
+size_t policy_sgd_smem_bytes(int K0, int h1, int h2, int A);
+size_t policy_sgd_scratch_floats(int K0, int h1, int h2, int A);
+cudaError_t launch_policy_sgd(const PolicySgdArgs& a, cudaStream_t s);
+// out = sum over rows of ll (SGD_BC_MLE) or sum over rows x A of (mu - act)^2 (SGD_BC_MSE); scratch >= 128 doubles
+cudaError_t launch_bc_loss_sum(const float* ll, const float* mu, const float* act, long long n, int A, int kind,
+                               double* scratch, double* out, cudaStream_t s);
+
 }  // namespace mjb

@@ -9,6 +9,7 @@
 // with feature-major activations in shared memory, and each thread Adam-updates the parameters whose
 // gradient it just accumulated in registers.  Weights live in global memory (L1/L2-resident, 78 KB) in
 // both natural and transposed form so every inner loop reads them coalesced.
+#include "adam.cuh"
 #include "kernels.h"
 
 namespace mjb {
@@ -16,17 +17,6 @@ namespace mjb {
 constexpr int VB = 64;             // max minibatch rows
 constexpr int VL = VB + 4;         // row pitch of feature-major activations
 constexpr int VT = 1024;           // threads
-
-struct AdamC { float one_m_b1, b2, one_m_b2, bc2_sqrt, eps, neg_step, reg; };
-
-__device__ __forceinline__ float adam_step(float g, float w, float* m, float* v, const AdamC& c) {
-    g = fmaf(c.reg, w, g);                               // grad.add(param, alpha=weight_decay)
-    const float mn = *m + c.one_m_b1 * (g - *m);         // exp_avg.lerp_(grad, 1-beta1)
-    const float vn = fmaf(c.one_m_b2 * g, g, *v * c.b2); // exp_avg_sq.mul_(beta2).addcmul_(g, g, 1-beta2)
-    *m = mn; *v = vn;
-    const float denom = sqrtf(vn) / c.bc2_sqrt + c.eps;
-    return fmaf(c.neg_step, mn / denom, w);              // param.addcdiv_(exp_avg, denom, value=-step_size)
-}
 
 // out4[n][4 samples q] = sum_k inT[k][4q..] * WT[k][n]   for unit o = n + NOUT*q
 __device__ __forceinline__ float4 dense_unit(const float* __restrict__ inT, const float* WT, int NOUT, int R, int n, int q) {

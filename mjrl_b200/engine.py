@@ -9,6 +9,7 @@ from . import _native
 from ._native import BatchStats, Config, MjbError, StepStats
 
 ALGO = {"npg": 0, "trpo": 1, "dapg": 2}
+LOSS = {"ppo": 0, "mle": 1, "mse": 2}
 ROLLOUT, DEMO = 0, 1
 
 
@@ -327,6 +328,47 @@ class Engine:
                                           int(cg_iters), float(damping), float(demo_lam), _ptr(ii),
                                           0 if ii is None else ii.shape[1], C.byref(st)), "policy_step")
         return st
+
+    # ------------------------------------------------------------------ minibatch-Adam policy training (PPO, BC)
+    def policy_sgd(self, loss, idx, lr, clip_coef=0.2, want_outputs=False):
+        """Sequential Adam steps on theta_new (csrc/policy_sgd.cu), one minibatch per row of idx [steps, batch] (rows of
+        the resident batch).  loss: "ppo", "mle" or "mse".  want_outputs: also return every step's minibatch loss and
+        (PPO) the fraction of the minibatch the clip zeroed, as two float32 arrays."""
+        ii = np.ascontiguousarray(idx, dtype=np.int32)
+        if ii.ndim != 2:
+            raise ValueError("policy_sgd: idx must be [steps, batch]")
+        steps, batch = ii.shape
+        if ii.size and (int(ii.min()) < 0 or int(ii.max()) >= self.n):
+            raise ValueError("policy_sgd: minibatch index outside the resident batch of %d rows" % self.n)
+        loss_out = np.empty(steps, np.float32) if want_outputs else None
+        clip_out = np.empty(steps, np.float32) if want_outputs else None
+        self._ck(self.lib.mjb_policy_sgd(self.h, LOSS[loss], _ptr(ii), int(steps), int(batch), float(lr), float(clip_coef),
+                                         _ptr(loss_out), _ptr(clip_out)), "policy_sgd")
+        return (loss_out, clip_out) if want_outputs else None
+
+    def adam_set(self, m=None, v=None, step=-1):
+        arrs = [None if a is None else _f32(a) for a in (m, v)]
+        for a in arrs:
+            assert a is None or a.shape[0] == self.d
+        self._ck(self.lib.mjb_policy_adam_set(self.h, _ptr(arrs[0]), _ptr(arrs[1]), int(step)), "policy_adam_set")
+
+    def adam_get(self):
+        m, v = np.empty(self.d, np.float32), np.empty(self.d, np.float32)
+        step = C.c_int64()
+        self._ck(self.lib.mjb_policy_adam_get(self.h, _ptr(m), _ptr(v), C.byref(step)), "policy_adam_get")
+        return m, v, int(step.value)
+
+    def bc_loss(self, loss):
+        """Full-batch BC loss ("mle" or "mse") of theta_new over the resident batch."""
+        out = C.c_double()
+        self._ck(self.lib.mjb_policy_bc_loss(self.h, LOSS[loss], C.byref(out)), "policy_bc_loss")
+        return float(out.value)
+
+    def last_sgd_ms(self):
+        """CUDA-event time of the last policy_sgd chain."""
+        t = C.c_float()
+        self._ck(self.lib.mjb_policy_sgd_timing(self.h, C.byref(t)), "policy_sgd_timing")
+        return float(t.value)
 
     def set_tensor_cores(self, on=True):
         """Returns True when the tcgen05 FVP path is active for this policy shape."""
